@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- rows/sec of the scoring hot path at batch = 65 536 x 23 features (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--model gbdt100d6|rf100d6]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--model gbdt100d6|rf100d6] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 One "step" = one pass of the hot path over one 65 536-row batch of synthetic credit-default rows
@@ -20,6 +20,11 @@ Printed by rank 0: ONE JSON line.
   cpu_baseline  the reference-style sklearn pipeline's predict_proba on this box's host cores (rank 0, N=1).
 
 --impl reference times that CPU path alone (all host cores, process pool) and prints the same line shape.
+
+--dump-outputs DIR  rank 0 writes what the last timed step of each timed path returned, as DIR/<name>.npy:
+  value_proba1.npy, value_label.npy   float32 (65 536,): probability of class 1 and label of the value path's last launch
+  e2e_predictions.npy                 float64 (65 536,): ``predictions`` of the plugin path's last B200Model.predict call
+  Inputs and models are seeded, so two builds run with the same arguments can be compared output for output.
 """
 
 from __future__ import annotations
@@ -30,6 +35,7 @@ import os
 import statistics
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -135,7 +141,8 @@ def get_pipeline(name: str, dist: Dist):
     from databricks_kubernetes_mlops_poc_b200 import training
 
     kind, params = MODELS[name]
-    cache_dir = os.environ.get("B2F_BENCH_CACHE", "/tmp/b2f_bench_cache")
+    # per user: on a shared host another user's directory of the same name is neither writable nor to be unpickled
+    cache_dir = os.environ.get("B2F_BENCH_CACHE", os.path.join(tempfile.gettempdir(), f"b2f_bench_cache_{os.getuid()}"))
     os.makedirs(cache_dir, exist_ok=True)
     n_train = N_TRAIN_BY_MODEL.get(name, N_TRAIN)
     path = os.path.join(cache_dir, f"{name}_n{n_train}_s{TRAIN_SEED}_sk{sklearn.__version__}.joblib")
@@ -431,6 +438,14 @@ def run_b200(args, dist: Dist):
     l0 = eng.info()["launches"]
     _, ms_total = eng.predict_stream_timed(d_rows, BATCH, POOL, d_proba, False, d_label, K, fmt=fmt, per_launch=False)
     launches_value = eng.info()["launches"] - l0
+    outputs = {}
+    if args.dump_outputs and dist.rank == 0:  # launch i scores pool batch i % POOL into its own slot of d_proba / d_label
+        last = (K - 1) % POOL
+        outputs["value_proba1"] = np.empty(BATCH, dtype=np.float32)
+        eng.d2h(outputs["value_proba1"], d_proba + last * BATCH * 4)
+        label = np.empty(BATCH, dtype=np.int32)
+        eng.d2h(label, d_label + last * BATCH * 4)
+        outputs["value_label"] = label.astype(np.float32)
     dist.barrier()
     ms_total_max = dist.max(ms_total)
     value = dist.world * BATCH * K / (ms_total_max * 1e-3)
@@ -518,6 +533,8 @@ def run_b200(args, dist: Dist):
         stages.append(model.last_timing)
     plugin_s = time.perf_counter() - t0
     launches_plugin = eng.info()["launches"] - l0
+    if args.dump_outputs and dist.rank == 0:
+        outputs["e2e_predictions"] = np.asarray(out0["predictions"], dtype=np.float64)
     dist.barrier()
     plugin_value = dist.world * BATCH * K / dist.max(plugin_s)
     st = [s for s in stages if s]
@@ -688,6 +705,11 @@ def run_b200(args, dist: Dist):
 
         if device_count() > 1:  # config 4 inside the default single-process run when the box shows several GPUs
             line["cfg4_stream"] = stream_leg(args, pipe, base, flat, rows_total=args.stream_rows, sustain=1.0)
+    if outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in outputs.items():
+            np.save(os.path.join(args.dump_outputs, f"{name}.npy"), a)
+        print(f"[bench] wrote {', '.join(f'{n}.npy' for n in outputs)} to {args.dump_outputs}", file=sys.stderr)
     if dist.rank == 0:
         emit(line)
 
@@ -999,7 +1021,11 @@ def main():
     ap.add_argument("--stream-rows", type=int, default=10_000_000)
     ap.add_argument("--quick", action="store_true", help="only the timed value / e2e legs (no sweep, stream, cpu baseline, outliers, drift)")
     ap.add_argument("--stream-gpus", type=int, default=0, help="GPUs used by --stream (0 = all visible)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs to DIR/<name>.npy (rank 0; see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.quick:
         args.no_sweep = args.no_stream = args.no_cpu = args.no_outliers = args.no_drift = args.no_gib = True
 

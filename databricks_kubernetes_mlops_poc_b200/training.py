@@ -111,8 +111,9 @@ def load_base_frame(path: str | None = None) -> pd.DataFrame:
         cols = {}
         for j, name in enumerate(CATEGORICAL_FEATURES):
             cols[name] = z[f"vocab_{j}"][z[f"codes_{j}"].astype(np.int64)].astype(object)
+        nums = z["nums_cents"] / 100.0  # stored as int32 hundredths; exact for the table's two-decimal values
         for k, name in enumerate(NUMERIC_FEATURES):
-            cols[name] = z["nums"][:, k]
+            cols[name] = nums[:, k]
         df = pd.DataFrame(cols)
         for name in CATEGORICAL_FEATURES:
             df[name] = df[name].astype(str)

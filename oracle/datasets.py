@@ -3,8 +3,10 @@
 ``tests/golden/curated.npz`` / ``inference.npz`` are lossless dictionary-encoded
 copies of the reference's ``databricks/data/curated.csv`` (30 000 labelled rows)
 and ``databricks/data/inference.csv`` (80 rows, different column order), written
-by ``tests/golden/make_golden.py``.  They exist because ``/root/reference`` is not
-present on the GPU box.
+by ``tests/golden/make_golden.py``, so that the tests need nothing outside the
+repository.  Every numeric value in those files has at most two decimals; it is
+stored as int32 hundredths (``nums_cents``), and ``cents / 100.0`` gives back the
+float64 the CSV parser produced, bit for bit.
 """
 
 from __future__ import annotations
@@ -23,8 +25,9 @@ def _thaw(z, with_target: bool) -> pd.DataFrame:
     cols = {}
     for j, name in enumerate(CATEGORICAL_FEATURES):
         cols[name] = z[f"vocab_{j}"][z[f"codes_{j}"].astype(np.int64)].astype(object)
+    nums = z["nums_cents"] / 100.0
     for j, name in enumerate(NUMERIC_FEATURES):
-        cols[name] = z["nums"][:, j]
+        cols[name] = nums[:, j]
     df = pd.DataFrame(cols)
     for name in CATEGORICAL_FEATURES:
         df[name] = df[name].astype(str)

@@ -39,7 +39,10 @@ def freeze_frame(df: pd.DataFrame, with_target: bool) -> dict:
         vocab, codes = np.unique(df[name].astype(str).to_numpy(), return_inverse=True)
         out[f"vocab_{j}"] = vocab.astype("U")
         out[f"codes_{j}"] = codes.astype(np.int8)
-    out["nums"] = df[rp.NUMERIC_FEATURES].to_numpy(dtype=np.float64)
+    # the CSV's numerics carry at most two decimals: int32 hundredths store them exactly in half the bytes of float64
+    nums = df[rp.NUMERIC_FEATURES].to_numpy(dtype=np.float64)
+    out["nums_cents"] = np.round(nums * 100.0).astype(np.int32)
+    assert (out["nums_cents"] / 100.0 == nums).all() and not (np.signbit(nums) & (nums == 0)).any()
     if with_target:
         out["target"] = df[rp.TARGET].to_numpy(dtype=np.int8)
     return out

@@ -3,7 +3,9 @@ configs[1]  GBDT 100 x depth 6 at the full 65 536-row synthetic batch -- every k
             labels exact on the WHOLE batch (not a sample);
 configs[2]  GBDT 500 x depth 8 and RF 500 x depth 8 at the latency-sweep sizes {1, 16, 256, 4096, 65536}."""
 
+import json
 import os
+import subprocess
 import sys
 
 import numpy as np
@@ -123,3 +125,31 @@ def test_cfg3_500d8_at_the_sweep_sizes(bench_mod, name):
             assert np.abs(np.asarray(out["predictions"]) - want_p[:n]).max() <= TOL64, (name, n)
     finally:
         model.close()
+
+
+def test_bench_dumps_the_last_timed_step(bench_mod, tmp_path):
+    """`bench.py --steps K --dump-outputs DIR`: K timed launches, and the dumped arrays are what the last of them (pool batch
+    (K - 1) % POOL) and the plugin path's last call returned -- each equal to sklearn on its own rows."""
+    from databricks_kubernetes_mlops_poc_b200 import training
+    from databricks_kubernetes_mlops_poc_b200.schema import ALL_FEATURES
+
+    K = 35  # the last launch scores pool batch 2, not batch 0
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--quick", "--no-moments", "--steps", str(K), "--warmup", "3",
+                        "--dump-outputs", str(tmp_path)], capture_output=True, text=True, cwd=ROOT, timeout=1800)
+    assert r.returncode == 0, r.stderr[-3000:]
+    line = json.loads(r.stdout.strip().splitlines()[-1])
+    assert line["steps"] == K and line["gpu_launches"] == K
+    assert sorted(os.listdir(tmp_path)) == ["e2e_predictions.npy", "value_label.npy", "value_proba1.npy"]
+    proba, label, e2e = (np.load(tmp_path / f"{n}.npy") for n in ("value_proba1", "value_label", "e2e_predictions"))
+    assert proba.dtype == label.dtype == np.float32 and e2e.dtype == np.float64
+    assert proba.shape == label.shape == e2e.shape == (bench_mod.BATCH,)
+
+    pipe, base = _model(bench_mod, "gbdt100d6")
+    last = (K - 1) % bench_mod.POOL
+    vocabs, codes, nums = training.synth_arrays(base, bench_mod.POOL * bench_mod.BATCH, bench_mod.DATA_SEED)
+    rows = slice(last * bench_mod.BATCH, (last + 1) * bench_mod.BATCH)
+    df = training.arrays_to_frame(vocabs, codes[rows], nums[rows])[ALL_FEATURES]
+    assert np.abs(proba.astype(np.float64) - pipe.predict_proba(df)[:, 1]).max() <= TOL32
+    assert (label == pipe.predict(df)).all()
+    _, _, df0 = _synthetic(bench_mod, base, bench_mod.BATCH, bench_mod.DATA_SEED)
+    assert np.abs(e2e - pipe.predict_proba(df0)[:, 1]).max() <= TOL64

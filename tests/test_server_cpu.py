@@ -105,43 +105,59 @@ def test_concurrent_requests_share_batches():
     assert sum(m.calls) == 120 and len(m.calls) < 40  # requests were merged into fewer engine calls
 
 
-REFERENCE_APP = "/root/reference/app"
-
-
-@pytest.mark.skipif(not __import__("os").path.exists(REFERENCE_APP + "/main.py"), reason="reference checkout not present (GPU box)")
-def test_unmodified_reference_app_runs_on_the_shim(monkeypatch):
-    """SURVEY 8f rank 4: the reference's own app/main.py, imported unmodified from /root/reference with the mlflow shim
-    ahead on the path, serves POST /predict from whatever `load_model` returns (a stub scorer here: no GPU)."""
-    import importlib
+def test_service_and_shim_match_the_recorded_reference_app(monkeypatch, curated):
+    """SURVEY 8f rank 4: the reference's own app/main.py, run unmodified on the mlflow shim, was recorded into
+    tests/golden/reference_app.json (make_golden_reference_app.py) with a stub scorer behind `load_model`.  The shim
+    must serve the `load_model` call that app made, and the project's app, given the same stub and the same request
+    bodies, must answer with the same statuses and responses, hand the model the same frames and log the same records."""
+    import importlib.util
+    import json
     import os
     import sys
 
     import databricks_kubernetes_mlops_poc_b200 as pkg
-    from databricks_kubernetes_mlops_poc_b200.schema import ALL_FEATURES, sample_request
+    from databricks_kubernetes_mlops_poc_b200.ingest import NATIVE_MIN_BYTES
+    from databricks_kubernetes_mlops_poc_b200.server import create_app
 
-    class Plugin:  # the plugin boundary: predict(DataFrame) -> dict (CustomModel.predict)
-        def predict(self, df):
-            if len(df.columns) == 0:
-                raise KeyError("no columns")  # what B200Model.predict (and the reference's CustomModel) do on []
-            n = len(df)
-            return {"predictions": [0.25] * n, "outliers": [0] * n, "feature_drift_batch": {k: 0.0 for k in ALL_FEATURES}}
+    golden_dir = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+    spec = importlib.util.spec_from_file_location("make_golden_reference_app", os.path.join(golden_dir, "make_golden_reference_app.py"))
+    rec = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(rec)
+    with open(rec.GOLDEN) as f:
+        golden = json.load(f)
+    bodies = rec.request_bodies(curated)
+    assert [name for name, _ in bodies] == [c["name"] for c in golden["cases"]]
+    assert len(bodies[-1][1]) > NATIVE_MIN_BYTES  # one body takes the native parser
 
-    monkeypatch.syspath_prepend(REFERENCE_APP)
-    monkeypatch.syspath_prepend(os.path.join(os.path.dirname(pkg.__file__), "shim"))
-    for name in [m for m in sys.modules if m in ("mlflow", "main", "model") or m.startswith("mlflow.")]:
+    model, load_calls = rec.StubModel(), []
+    monkeypatch.setattr(pkg, "load_model", lambda path, **kw: (load_calls.append(path), model)[1])
+    for var in ("MODEL_DIRECTORY", "SERVICE_NAME"):
+        monkeypatch.delenv(var, raising=False)
+
+    monkeypatch.syspath_prepend(rec.SHIM)
+    for name in [m for m in sys.modules if m == "mlflow" or m.startswith("mlflow.")]:
         monkeypatch.delitem(sys.modules, name)
-    monkeypatch.setattr(pkg, "load_model", lambda path: Plugin())
-    main = importlib.import_module("main")
     try:
-        assert main.__file__.startswith(REFERENCE_APP)
-        with TestClient(main.app, raise_server_exceptions=False) as c:
-            r = c.post("/predict", json=sample_request())
-            assert r.status_code == 200 and r.json()["predictions"] == [0.25]
-            assert list(r.json()["feature_drift_batch"]) == ALL_FEATURES
-            assert c.post("/predict", json=[]).status_code == 500
+        import mlflow
+
+        assert mlflow.__file__.startswith(rec.SHIM)
+        for path in golden["load_model_calls"]:
+            assert mlflow.pyfunc.load_model(path) is model
+        assert load_calls == golden["load_model_calls"]
     finally:
-        for name in [m for m in sys.modules if m in ("mlflow", "main", "model") or m.startswith("mlflow.")]:
+        for name in [m for m in sys.modules if m == "mlflow" or m.startswith("mlflow.")]:
             sys.modules.pop(name, None)
+
+    load_calls.clear()
+    with rec.captured_log_records() as records, TestClient(create_app(), raise_server_exceptions=False) as c:
+        got = rec.replay(c, bodies, model, records)
+    assert load_calls == golden["load_model_calls"]  # lifespan loads from the same default path
+    for g, want in zip(got, golden["cases"]):
+        assert g["status"] == want["status"], g["name"]
+        if "response" in g:  # the reference's response model renders the 0 / 1 outlier flags as 0.0 / 1.0, the project as 0 / 1
+            g["response"]["outliers"] = [float(v) for v in g["response"]["outliers"]]
+        # everything else exactly, keys in order (json.dumps tells -0.0 from 0.0 and 1 from 1.0)
+        assert json.dumps(g) == json.dumps(want), g["name"]
 
 
 def test_one_pass_request_parsing_equals_the_model_validation():
