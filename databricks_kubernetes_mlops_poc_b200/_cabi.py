@@ -70,7 +70,7 @@ class Info(C.Structure):
         ("rank_smem_bytes", C.c_int32),
         ("rank_row_bytes", C.c_int32),
         ("rank_stream", C.c_int32),
-        ("reserved2", C.c_int32),
+        ("rank_last_pdl", C.c_int32),
     ]
 
 

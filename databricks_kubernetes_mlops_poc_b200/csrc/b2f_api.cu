@@ -18,9 +18,12 @@
 #include <string.h>
 
 #include <algorithm>
+#include <deque>
+#include <mutex>
 #include <string>
 #include <thread>
 #include <new>
+#include <unordered_map>
 #include <vector>
 
 #include "../../include/b2f.h"
@@ -160,6 +163,10 @@ struct b2f_model {
     int rank_u = 4;
     bool rank_stream = false; /* the rank layout streams through shared memory in pieces (too large to stay resident) */
     int64_t launches_rank = 0;
+    bool rank_last_pdl = false; /* the last rank launch went out with programmatic stream serialization */
+#ifdef B2F_RANK_TRACE
+    unsigned long long *d_rank_trace = nullptr; /* B2F_RANK_TRACE_LAUNCHES launches x sm_count CTAs x B2F_RANK_TRACE_WORDS */
+#endif
     void *d_blob = nullptr;
     int64_t forest_bytes = 0;
     b2f_model *outlier = nullptr; /* attached isolation forest (b2f_model_attach_outlier_forest): a child handle on the
@@ -186,6 +193,53 @@ struct b2f_model {
     int rank = 0;
     int64_t launches = 0;
 };
+
+/* the rank kernel goes out with programmatic stream serialization: back-to-back launches on one stream overlap the next
+ * launch's prologue (forest fill, row staging) with this launch's tail.  The kernel waits (griddepcontrol.wait) only before its
+ * first global store, so it reads its rows while earlier launches may still run -- not only the previous one: every rank launch
+ * triggers its dependents at entry, so a chain of launches with the attribute can be resident at once (small grids leave SMs
+ * free).  A launch whose rows overlap what any launch of the current chain writes therefore goes out without the attribute;
+ * it starts only after its predecessor has completed, which completed only after its own wait, i.e. after everything before
+ * it: such a launch starts a new chain.
+ * How far back a chain must be remembered: a CTA passes its wait only after the previous launch has completed, and every CTA
+ * passes it before it exits, so while launch A is incomplete every later launch of the chain holds a resident CTA (all of its
+ * CTAs have started: the launch after it has).  At most 2 rank CTAs (1024 threads each) fit an SM, so when a new launch starts,
+ * a launch more than 2 * sm_count + 1 launches back has completed and a later launch has waited for it (its writes are
+ * flushed): the record keeps the chain's last 2 * sm_count + 1 launches and drops older ones.  Per stream (models share
+ * streams: an attached outlier forest runs on its parent's). */
+struct RankWrites {
+    uintptr_t p0, p1, l0, l1; /* proba [p0, p1), label [l0, l1) */
+};
+static std::mutex g_rank_writes_mu;
+static std::unordered_map<cudaStream_t, std::deque<RankWrites>> g_rank_writes;
+
+static bool rank_launch_pdl(cudaStream_t st, int sm_count, const void *rows, size_t rows_bytes, const void *proba, size_t psz, const int32_t *label,
+                            int64_t n, int ostride) {
+    static const bool no_pdl = getenv("B2F_NO_PDL") != nullptr;
+    const int64_t ps = ostride & 0xffff, ls = (ostride >> 16) ? (ostride >> 16) : ps; /* ostride_p / ostride_l */
+    RankWrites w;
+    w.p0 = reinterpret_cast<uintptr_t>(proba);
+    w.p1 = proba ? w.p0 + (size_t)((n - 1) * ps + 1) * psz : w.p0;
+    w.l0 = reinterpret_cast<uintptr_t>(label);
+    w.l1 = label ? w.l0 + (size_t)((n - 1) * ls + 1) * sizeof(int32_t) : w.l0;
+    const uintptr_t r0 = reinterpret_cast<uintptr_t>(rows), r1 = r0 + rows_bytes;
+    std::lock_guard<std::mutex> lk(g_rank_writes_mu);
+    std::deque<RankWrites> &chain = g_rank_writes[st];
+    bool pdl = !no_pdl;
+    for (const RankWrites &c : chain)
+        if ((c.p0 < r1 && r0 < c.p1) || (c.l0 < r1 && r0 < c.l1)) {
+            pdl = false;
+            break;
+        }
+    if (!pdl) chain.clear();
+    chain.push_back(w);
+    while (chain.size() > 2 * (size_t)sm_count + 1) chain.pop_front();
+    return pdl;
+}
+static void rank_forget_stream(cudaStream_t st) {
+    std::lock_guard<std::mutex> lk(g_rank_writes_mu);
+    g_rank_writes.erase(st);
+}
 
 static int validate_blob(const uint8_t *blob, size_t nbytes, b2f_blob_header *hdr_out) {
     if (!blob || nbytes < sizeof(b2f_blob_header)) return set_err(B2F_EINVAL, "forest blob too small (%zu bytes)", nbytes);
@@ -467,31 +521,50 @@ static int rank_init(b2f_model *m, const uint8_t *blob) {
     const char *off = getenv("B2F_RANK");
     if (off && !strcmp(off, "0")) return B2F_OK;
     const int64_t layout_bytes = (int64_t)m->rk.layout.size();
+    /* resident: the per-group head table (rank_walk_group_head) follows the trees, 3U words per group of U trees */
+    const int64_t head_bytes = (int64_t)m->rk.n_trees_padded * 12;
     const int64_t base = B2F_RANK_XS_BYTES /* alignment slack */ + (int64_t)B2F_RANK_PARTIALS * 32 * 8 + 256;
-    int max_tiles = (int)std::min<int64_t>(B2F_RANK_MAX_TILES, ((int64_t)m->max_smem_optin - base - layout_bytes) / B2F_RANK_XS_BYTES);
+    int max_tiles = (int)std::min<int64_t>(B2F_RANK_MAX_TILES, ((int64_t)m->max_smem_optin - base - layout_bytes - head_bytes) / B2F_RANK_XS_BYTES);
     if (const char *mt = getenv("B2F_RANK_MAX_TILES")) max_tiles = std::min(max_tiles, std::max(1, atoi(mt)));
     /* resident while the whole layout fits next to a useful number of row tiles; otherwise it streams through a two-slot ring
      * in pieces of 8 trees (2 groups of 4: warp w owns (tile w / 2, group w mod 2), so <= 16 tiles per round) */
     m->rank_stream = max_tiles < 8;
     if (const char *fs = getenv("B2F_RANK_STREAM")) m->rank_stream = atoi(fs) != 0;
-    int64_t forest_smem = layout_bytes;
+    int64_t forest_smem = layout_bytes + head_bytes;
     m->rank_u = 4;
     if (const char *ru = getenv("B2F_RANK_U")) m->rank_u = atoi(ru) == 8 ? 8 : 4;
+    std::vector<uint8_t> dev_layout(m->rk.layout);
     if (m->rank_stream) {
         m->rank_u = 4;
         const int64_t piece = 8 * (int64_t)m->rk.tree_stride; /* n_trees_padded is a multiple of 8 */
         forest_smem = 2 * piece;
         max_tiles = (int)std::min<int64_t>(B2F_RANK_MAX_TILES, ((int64_t)m->max_smem_optin - base - forest_smem) / B2F_RANK_XS_BYTES);
         if (max_tiles < 4 || piece % 16) return B2F_OK;
+    } else {
+        const int U = m->rank_u, n_nodes = 1 << m->rk.depth;
+        std::vector<uint32_t> head((size_t)head_bytes / 4, 0u);
+        for (int t = 0; t < m->rk.n_trees_padded; ++t) {
+            const uint32_t *nodes = reinterpret_cast<const uint32_t *>(m->rk.layout.data() + (size_t)t * m->rk.tree_stride);
+            uint32_t *g = head.data() + (size_t)(t / U) * 3 * U;
+            g[t % U] = nodes[0];
+            if (n_nodes > 2) { /* depth 1: no level 1 (node word 1 is the unused last one) */
+                g[U + 2 * (t % U)] = nodes[1];
+                g[U + 2 * (t % U) + 1] = nodes[2];
+            }
+        }
+        dev_layout.resize((size_t)(layout_bytes + head_bytes));
+        memcpy(dev_layout.data() + layout_bytes, head.data(), (size_t)head_bytes);
     }
-    CUDA_TRY(cudaMalloc(&m->d_rank_layout, (size_t)layout_bytes));
-    CUDA_TRY(cudaMemcpy(m->d_rank_layout, m->rk.layout.data(), (size_t)layout_bytes, cudaMemcpyHostToDevice));
+    CUDA_TRY(cudaMalloc(&m->d_rank_layout, dev_layout.size()));
+    CUDA_TRY(cudaMemcpy(m->d_rank_layout, dev_layout.data(), dev_layout.size(), cudaMemcpyHostToDevice));
     RParams &rp = m->rp;
     memset(&rp, 0, sizeof(rp));
     rp.layout = static_cast<const uint8_t *>(m->d_rank_layout);
-    rp.layout_bytes = (uint32_t)layout_bytes;
+    rp.layout_bytes = (uint32_t)dev_layout.size();
     rp.tree_stride = m->rk.tree_stride;
     rp.n_trees_padded = m->rk.n_trees_padded;
+    rp.n_groups = (m->rk.n_trees + m->rank_u - 1) / m->rank_u;
+    rp.head_off = (uint32_t)layout_bytes;
     rp.depth = m->rk.depth;
     rp.agg_mode = (int)m->hdr.agg_mode;
     rp.n_cat = m->rk.n_cat;
@@ -520,6 +593,11 @@ static int rank_init(b2f_model *m, const uint8_t *blob) {
         rp.cat_start[j] = (uint8_t)i;
         rp.cat_mask[j] |= 1ull << c;
     }
+#ifdef B2F_RANK_TRACE
+    const size_t trace_bytes = (size_t)B2F_RANK_TRACE_LAUNCHES * m->sm_count * B2F_RANK_TRACE_WORDS * sizeof(unsigned long long);
+    CUDA_TRY(cudaMalloc(&m->d_rank_trace, trace_bytes));
+    CUDA_TRY(cudaMemset(m->d_rank_trace, 0, trace_bytes));
+#endif
     m->rank_smem_bytes = (int)(B2F_RANK_XS_BYTES + (int64_t)max_tiles * B2F_RANK_XS_BYTES + (int64_t)B2F_RANK_PARTIALS * 32 * 8 + forest_smem);
     if (m->rank_stream)
         CUDA_TRY((rank_set_attr_all<4, true>(rp.depth, m->rank_smem_bytes)));
@@ -733,16 +811,25 @@ extern "C" void b2f_model_destroy(b2f_model *m) {
         if (sl.d_rows) cudaFree(sl.d_rows);
         if (sl.d_proba) cudaFree(sl.d_proba);
         if (sl.d_label) cudaFree(sl.d_label);
-        if (sl.stream) cudaStreamDestroy(sl.stream);
+        if (sl.stream) {
+            rank_forget_stream(sl.stream);
+            cudaStreamDestroy(sl.stream);
+        }
     }
     for (auto &t : m->tickets)
         for (auto &e : t.ev)
             if (e) cudaEventDestroy(e);
-    if (m->compute) cudaStreamDestroy(m->compute);
+    if (m->compute) {
+        rank_forget_stream(m->compute);
+        cudaStreamDestroy(m->compute);
+    }
     if (m->d_blob) cudaFree(m->d_blob);
     if (m->d_tile_layout) cudaFree(m->d_tile_layout);
     if (m->d_tile_pieces) cudaFree(m->d_tile_pieces);
     if (m->d_rank_layout) cudaFree(m->d_rank_layout);
+#ifdef B2F_RANK_TRACE
+    if (m->d_rank_trace) cudaFree(m->d_rank_trace);
+#endif
     if (m->d_mom_rows) cudaFree(m->d_mom_rows);
     if (m->d_mom_partials) cudaFree(m->d_mom_partials);
     if (m->d_mom_ticket) cudaFree(m->d_mom_ticket);
@@ -790,6 +877,7 @@ extern "C" int b2f_model_info(const b2f_model *m, b2f_info *out) {
     out->rank_smem_bytes = m->rank_ok ? m->rank_smem_bytes : 0;
     out->rank_row_bytes = m->rk.row_bytes;
     out->rank_stream = (m->rank_ok && m->rank_stream) ? 1 : 0;
+    out->rank_last_pdl = m->rank_last_pdl ? 1 : 0;
     return B2F_OK;
 }
 
@@ -843,10 +931,9 @@ static cudaError_t launch_split(const b2f_model *m, cudaStream_t st, const void 
     return cudaGetLastError();
 }
 
-/* the rank kernel goes out with programmatic stream serialization: back-to-back launches on one stream overlap the
- * next launch's prologue (forest fill) with this launch's tail; the kernel orders its own global accesses with griddepcontrol.wait */
+/* the rank kernel goes out with programmatic stream serialization (see rank_launch_pdl) */
 template <int D, int U, bool ST, typename OutT>
-static cudaError_t launch_rank_du(const b2f_model *m, cudaStream_t st, const void *rows, int64_t n, void *proba, int32_t *label, int ostride) {
+static cudaError_t launch_rank_du(const b2f_model *m, cudaStream_t st, const void *rows, int64_t n, void *proba, int32_t *label, int ostride, bool pdl) {
     const int64_t n_tiles = (n + 31) / 32;
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3((unsigned)std::max<int64_t>(1, std::min<int64_t>(m->sm_count, n_tiles)));
@@ -856,19 +943,39 @@ static cudaError_t launch_rank_du(const b2f_model *m, cudaStream_t st, const voi
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
-    static const bool no_pdl = getenv("B2F_NO_PDL") != nullptr;
     cfg.attrs = attr;
-    cfg.numAttrs = no_pdl ? 0 : 1;
-    return cudaLaunchKernelEx(&cfg, k_forest_predict_rank<D, U, ST, OutT>, m->rp, static_cast<const uint8_t *>(rows), (long long)n,
+    cfg.numAttrs = pdl ? 1 : 0;
+#ifdef B2F_RANK_TRACE
+    RParams rp = m->rp; /* launch i records into slot i mod B2F_RANK_TRACE_LAUNCHES */
+    rp.trace = m->d_rank_trace + (size_t)(m->launches_rank % B2F_RANK_TRACE_LAUNCHES) * m->sm_count * B2F_RANK_TRACE_WORDS;
+#else
+    const RParams &rp = m->rp;
+#endif
+    return cudaLaunchKernelEx(&cfg, k_forest_predict_rank<D, U, ST, OutT>, rp, static_cast<const uint8_t *>(rows), (long long)n,
                               static_cast<OutT *>(proba), label, ostride);
 }
+
+#ifdef B2F_RANK_TRACE
+/* traced build only: copy the trace ring (B2F_RANK_TRACE_LAUNCHES x sm_count x B2F_RANK_TRACE_WORDS words) to the host after
+ * a synchronise; returns the rank launches made so far (launch i sits in slot i mod B2F_RANK_TRACE_LAUNCHES) */
+extern "C" int64_t b2f_rank_trace_read(b2f_model *m, unsigned long long *out, int32_t *launch_slots, int32_t *ctas_per_launch) {
+    if (!m || !out || !m->d_rank_trace) return -1;
+    if (cudaSetDevice(m->device) != cudaSuccess || cudaDeviceSynchronize() != cudaSuccess) return -1;
+    if (cudaMemcpy(out, m->d_rank_trace, (size_t)B2F_RANK_TRACE_LAUNCHES * m->sm_count * B2F_RANK_TRACE_WORDS * sizeof(unsigned long long),
+                   cudaMemcpyDeviceToHost) != cudaSuccess)
+        return -1;
+    *launch_slots = B2F_RANK_TRACE_LAUNCHES;
+    *ctas_per_launch = m->sm_count;
+    return m->launches_rank;
+}
+#endif
 template <typename OutT>
-static cudaError_t launch_rank(const b2f_model *m, cudaStream_t st, const void *rows, int64_t n, void *proba, int32_t *label, int ostride) {
+static cudaError_t launch_rank(const b2f_model *m, cudaStream_t st, const void *rows, int64_t n, void *proba, int32_t *label, int ostride, bool pdl) {
 #define RK_CASE(DD)                                                                                                  \
     case DD:                                                                                                         \
-        if (m->rank_stream) return launch_rank_du<DD, 4, true, OutT>(m, st, rows, n, proba, label, ostride);          \
-        return m->rank_u == 8 ? launch_rank_du<DD, 8, false, OutT>(m, st, rows, n, proba, label, ostride)             \
-                              : launch_rank_du<DD, 4, false, OutT>(m, st, rows, n, proba, label, ostride);
+        if (m->rank_stream) return launch_rank_du<DD, 4, true, OutT>(m, st, rows, n, proba, label, ostride, pdl);     \
+        return m->rank_u == 8 ? launch_rank_du<DD, 8, false, OutT>(m, st, rows, n, proba, label, ostride, pdl)        \
+                              : launch_rank_du<DD, 4, false, OutT>(m, st, rows, n, proba, label, ostride, pdl);
     switch (m->rp.depth) {
         RK_CASE(1) RK_CASE(2) RK_CASE(3) RK_CASE(4) RK_CASE(5) RK_CASE(6) RK_CASE(7) RK_CASE(8)
     }
@@ -899,10 +1006,13 @@ static int launch_predict(b2f_model *m, cudaStream_t st, const void *rows_dev, i
     const bool pk = fmt == B2F_ROWS_PACKED64;
     cudaError_t e;
     if (fmt == B2F_ROWS_RANKED) { /* ranked rows have one kernel: integer compares on the resident rank layout */
-        e = f64 ? launch_rank<double>(m, st, rows_dev, n, proba_dev, label_dev, ostride) : launch_rank<float>(m, st, rows_dev, n, proba_dev, label_dev, ostride);
+        const bool pdl = rank_launch_pdl(st, m->sm_count, rows_dev, (size_t)n * (size_t)m->rk.row_bytes, proba_dev, f64 ? sizeof(double) : sizeof(float), label_dev, n, ostride);
+        e = f64 ? launch_rank<double>(m, st, rows_dev, n, proba_dev, label_dev, ostride, pdl)
+                : launch_rank<float>(m, st, rows_dev, n, proba_dev, label_dev, ostride, pdl);
         if (e != cudaSuccess) return set_err(B2F_ECUDA, "k_forest_predict_rank launch failed: %s", cudaGetErrorString(e));
         m->launches++;
         m->launches_rank++;
+        m->rank_last_pdl = pdl;
         return B2F_OK;
     }
     if (m->tile_ok && n >= m->tile_min_rows) {

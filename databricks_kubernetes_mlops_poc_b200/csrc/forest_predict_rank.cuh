@@ -21,9 +21,11 @@
  *              TRANSPOSED: lane l's values sit in bank l, so the per-lane dynamic fetch of the walk is one conflict-free
  *              LDS.U16), one lane per row and a share of the pseudo-features per thread, while one thread streams the forest
  *              into shared memory with TMA bulk copies (cp.async.bulk + mbarrier complete_tx);
- *   - phase 2  the round's work is tiles x tree groups (U trees per group, walked as U independent chains per thread); warp w
- *              takes the contiguous share [w * units / 32, (w+1) * units / 32) -- balanced to one tree group whatever the batch
- *              size -- and leaves one float64 partial per (warp, tile) it touched;
+ *   - phase 2  the round's work is tiles x tree groups (U trees per group, walked as U independent chains per thread; only the
+ *              ceil(n_trees / U) groups that hold real trees); warp w takes the contiguous share [w * units / 32, (w+1) * units / 32)
+ *              -- balanced to one tree group whatever the batch size -- and leaves one float64 partial per (warp, tile) it touched.
+ *              The top two levels of a group come from its head record (RParams::head_off): 3U words that every lane needs, read
+ *              as broadcast LDS.128, so a tree costs D - 2 per-lane node loads instead of D;
  *   - phase 3  one thread per row adds that row's partials in warp order (fixed order: deterministic), aggregates
  *              (RF mean | GBDT expit | isolation-forest score) and stores probability + label, coalesced.
  *   - STREAM = true (rank layouts larger than shared memory, e.g. 500 trees x depth 8 = 1.5 MB): the layout is cut into pieces of
@@ -31,8 +33,10 @@
  *     barrier that ends piece k, so the copy overlaps the walk of piece k + 1 -- and warp w owns (tile w / 2, group w mod 2) of
  *     EVERY piece: its float64 sum stays in a register across the whole forest (<= 16 tiles per round).
  *   - launched with programmatic stream serialization (PDL): `griddepcontrol.launch_dependents` is issued at entry so the next
- *     launch's CTAs take over SMs as this launch's CTAs retire (its forest fill and row staging overlap this launch's tail);
- *     `griddepcontrol.wait` sits before the first global access that could depend on the previous kernel.
+ *     launch's CTAs take over SMs as this launch's CTAs retire; `griddepcontrol.wait` sits before the first global STORE (phase 3),
+ *     so forest fill, row staging and the walk all overlap the previous launch's tail.  Reading rows before the wait is safe
+ *     because the host launches without PDL whenever the rows overlap the outputs of any rank launch still chained to this
+ *     one through PDL on that stream (b2f_api.cu rank_launch_pdl), and no other kernel triggers its dependents early.
  */
 #pragma once
 #include <cuda_runtime.h>
@@ -48,10 +52,13 @@
 #define B2F_RANK_PARTIALS (B2F_RANK_WARPS + B2F_RANK_MAX_TILES)
 
 struct RParams {
-    const uint8_t *layout;   /* device: n_trees_padded complete trees, tree_stride bytes each */
-    uint32_t layout_bytes;   /* multiple of 16 */
+    const uint8_t *layout;   /* device: n_trees_padded complete trees, tree_stride bytes each; resident: then the head table */
+    uint32_t layout_bytes;   /* multiple of 16 (resident: trees + head table) */
     uint32_t tree_stride;    /* 2^D * 12 */
     int32_t n_trees_padded;  /* multiple of 8 */
+    int32_t n_groups;        /* resident: tree groups walked per tile = ceil(n_trees / U) (the stub trees past them add 0.0) */
+    uint32_t head_off;       /* resident: byte offset of the head table, 3U words per group of U trees: the U root words, then
+                                the U (left, right) level-1 word pairs (16-byte aligned, so a group's heads are 3U/4 LDS.128) */
     int32_t depth;
     int32_t agg_mode;
     int32_t n_cat;
@@ -73,7 +80,37 @@ struct RParams {
     uint8_t cat_bits[16];
     uint8_t cat_start[16];   /* pair index of feature j's first tested category (pairs are sorted by feature, then category) */
     unsigned long long cat_mask[16]; /* bit c set: category c of feature j is tested by some node */
+#ifdef B2F_RANK_TRACE
+    unsigned long long *trace; /* B2F_RANK_TRACE_WORDS words per CTA of this launch (see RANK_TRACE below) */
+#endif
 };
+
+/* B2F_RANK_TRACE (off in the normal build; tools/rank_phases.py builds a traced copy): thread 0 of every CTA records its SM
+ * and %globaltimer at the kernel's phase boundaries, so the time between launches can be split into phases */
+#define B2F_RANK_TRACE_WORDS 8
+#define B2F_RANK_TRACE_LAUNCHES 256
+enum { RT_SMID, RT_ENTRY, RT_FOREST, RT_WAIT, RT_STAGED, RT_WALKED, RT_EXIT };
+#ifdef B2F_RANK_TRACE
+__device__ __forceinline__ unsigned long long rank_trace_now() {
+    unsigned long long t;
+    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
+    return t;
+}
+__device__ __forceinline__ unsigned long long rank_trace_smid() {
+    uint32_t s;
+    asm volatile("mov.u32 %0, %%smid;" : "=r"(s));
+    return s;
+}
+#define RANK_TRACE(i)                                                                                                       \
+    do {                                                                                                                    \
+        if (threadIdx.x == 0)                                                                                               \
+            p.trace[(size_t)blockIdx.x * B2F_RANK_TRACE_WORDS + (i)] = (i) == RT_SMID ? rank_trace_smid() : rank_trace_now(); \
+    } while (0)
+#else
+#define RANK_TRACE(i) \
+    do {              \
+    } while (0)
+#endif
 
 __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
@@ -84,21 +121,14 @@ __device__ __forceinline__ uint32_t lds_u16(uint32_t a) {
     return v;
 }
 
-/* walk U consecutive trees (first tree at shared address t0) for this lane's row; payloads are added in tree order.
- * A chain keeps the ABSOLUTE shared address a = B + 4i of its node (B = the tree's base): the child 2i+1 (+1) sits at
- * 2a - B + 4 (+4), i.e. one SEL between the two per-tree constants (4 - B, 8 - B) and one multiply-add (FMA pipe). */
-template <int D, int U>
-__device__ __forceinline__ void rank_walk_group(uint32_t t0, uint32_t tree_stride, uint32_t xs_lane, uint32_t m2, uint32_t m64k, uint32_t a64k,
-                                                double &acc) {
-    uint32_t at[U], k4[U], k8[U];
+/* levels D0 .. D-1 of U chains, then the payloads (added in tree order).  A chain keeps the ABSOLUTE shared address a = B + 4i of
+ * its node (B = the tree's base): the child 2i+1 (+1) sits at 2a - B + 4 (+4), i.e. one SEL between the two per-tree constants
+ * (k4 = 4 - B, k8 = 8 - B) and one multiply-add (FMA pipe). */
+template <int D0, int D, int U>
+__device__ __forceinline__ void rank_walk_levels(uint32_t (&at)[U], const uint32_t (&k4)[U], const uint32_t (&k8)[U], uint32_t xs_lane, uint32_t m2,
+                                                 uint32_t m64k, uint32_t a64k, double &acc) {
 #pragma unroll
-    for (int u = 0; u < U; ++u) {
-        at[u] = t0 + u * tree_stride;
-        k4[u] = 4u - at[u];
-        k8[u] = 8u - at[u];
-    }
-#pragma unroll
-    for (int d = 0; d < D; ++d) {
+    for (int d = D0; d < D; ++d) {
 #pragma unroll
         for (int u = 0; u < U; ++u) {
             const uint32_t nw = lds32(at[u]);
@@ -110,6 +140,50 @@ __device__ __forceinline__ void rank_walk_group(uint32_t t0, uint32_t tree_strid
     /* a = B + 4 (2^D - 1 + leaf): payload at B + 4 * 2^D + 8 * leaf = 2a - B - 4 * 2^D + 8 = (a + a + k4) + (4 - 4 * 2^D) */
 #pragma unroll
     for (int u = 0; u < U; ++u) acc += lds_f64(at[u] + at[u] + k4[u] + 4u - (4u << D));
+}
+
+/* walk U consecutive trees (first tree at shared address t0) for this lane's row, every level from the tree body (streamed pieces) */
+template <int D, int U>
+__device__ __forceinline__ void rank_walk_group(uint32_t t0, uint32_t tree_stride, uint32_t xs_lane, uint32_t m2, uint32_t m64k, uint32_t a64k,
+                                                double &acc) {
+    uint32_t at[U], k4[U], k8[U];
+#pragma unroll
+    for (int u = 0; u < U; ++u) {
+        at[u] = t0 + u * tree_stride;
+        k4[u] = 4u - at[u];
+        k8[u] = 8u - at[u];
+    }
+    rank_walk_levels<0, D, U>(at, k4, k8, xs_lane, m2, m64k, a64k, acc);
+}
+
+/* the same walk with the top two levels taken from the group's head record (shared address hd): its 3U words are the same for
+ * every lane, so they arrive as 3U/4 broadcast LDS.128 instead of 2U per-lane node loads; the root test SELects the level-1 word */
+template <int D, int U>
+__device__ __forceinline__ void rank_walk_group_head(uint32_t t0, uint32_t hd, uint32_t tree_stride, uint32_t xs_lane, uint32_t m2, uint32_t m64k,
+                                                     uint32_t a64k, double &acc) {
+    static_assert(U % 4 == 0, "head records are read 4 words at a time");
+    uint32_t hw[3 * U];
+#pragma unroll
+    for (int q = 0; q < 3 * U / 4; ++q)
+        asm volatile("ld.shared.v4.u32 {%0, %1, %2, %3}, [%4];"
+                     : "=r"(hw[4 * q]), "=r"(hw[4 * q + 1]), "=r"(hw[4 * q + 2]), "=r"(hw[4 * q + 3])
+                     : "r"(hd + 16u * q));
+    uint32_t at[U], k4[U], k8[U];
+#pragma unroll
+    for (int u = 0; u < U; ++u) {
+        at[u] = t0 + u * tree_stride;
+        k4[u] = 4u - at[u];
+        k8[u] = 8u - at[u];
+        const uint32_t r = hw[u];
+        const bool c0 = lds_u16(xs_lane | (r & 0x1F82u)) * m64k + a64k >= r;
+        at[u] = at[u] * m2 + (c0 ? k8[u] : k4[u]); /* node 1 or 2 */
+        if constexpr (D >= 2) {
+            const uint32_t n1 = c0 ? hw[U + 2 * u + 1] : hw[U + 2 * u];
+            const bool c1 = lds_u16(xs_lane | (n1 & 0x1F82u)) * m64k + a64k >= n1;
+            at[u] = at[u] * m2 + (c1 ? k8[u] : k4[u]); /* node 3 .. 6 */
+        }
+    }
+    rank_walk_levels<(D >= 2 ? 2 : 1), D, U>(at, k4, k8, xs_lane, m2, m64k, a64k, acc);
 }
 
 template <int D, int U, bool STREAM, typename OutT>
@@ -124,6 +198,8 @@ __global__ void __launch_bounds__(B2F_RANK_THREADS, 1)
     const int warp = tid >> 5;
 
     pdl_launch_dependents(); /* the next launch may start filling SMs as this one's CTAs retire */
+    RANK_TRACE(RT_SMID);
+    RANK_TRACE(RT_ENTRY);
 
     /* shared-memory plan: [xs: max_tiles x 8 KB value blocks, 8 KB aligned][partials][forest | two-slot piece ring] */
     const uint32_t pad = (B2F_RANK_XS_BYTES - (smem_addr(smem) & (B2F_RANK_XS_BYTES - 1u))) & (B2F_RANK_XS_BYTES - 1u);
@@ -157,12 +233,11 @@ __global__ void __launch_bounds__(B2F_RANK_THREADS, 1)
     const uint32_t tq = n_tiles / gridDim.x, tr = n_tiles % gridDim.x;
     const uint32_t tile0 = blockIdx.x * tq + min(blockIdx.x, tr), cta_tiles = tq + (blockIdx.x < tr ? 1u : 0u);
     const uint32_t n_rounds = (cta_tiles + (uint32_t)p.max_tiles - 1u) / (uint32_t)p.max_tiles;
-    const int groups = p.n_trees_padded / U; /* tree groups per tile */
+    const int groups = p.n_groups; /* tree groups per tile (resident) */
     const uint32_t forest_addr = smem_addr(forest);
     const uint32_t xs_addr = smem_addr(xs_all);
+    const uint32_t head_addr = forest_addr + p.head_off;
     bool forest_ready = false;
-
-    pdl_wait(); /* rows may have been produced by the previous kernel in the stream; outputs may still be read by it */
 
     for (uint32_t round = 0; round < n_rounds; ++round) {
         const uint32_t rt0 = cta_tiles * round / n_rounds, rt1 = cta_tiles * (round + 1u) / n_rounds;
@@ -215,11 +290,13 @@ __global__ void __launch_bounds__(B2F_RANK_THREADS, 1)
             }
         }
         __syncthreads();
+        RANK_TRACE(RT_STAGED);
         if constexpr (!STREAM) {
             if (!forest_ready) {
                 mbar_wait(&forest_bar[0], 0);
                 forest_ready = true;
             }
+            RANK_TRACE(RT_FOREST);
         }
 
         if constexpr (STREAM) {
@@ -238,6 +315,9 @@ __global__ void __launch_bounds__(B2F_RANK_THREADS, 1)
             }
             if (mine) partial[warp * 32 + lane] = acc;
             __syncthreads();
+            RANK_TRACE(RT_WALKED);
+            pdl_wait(); /* before the first global store: see phase 3 of the resident path */
+            RANK_TRACE(RT_WAIT);
             for (int r = tid; r < n_rows; r += B2F_RANK_THREADS) {
                 const int t = r >> 5, ln = r & 31;
                 double s = p.agg_mode == B2F_AGG_GBDT_LOGISTIC ? p.init_raw : 0.0;
@@ -263,12 +343,20 @@ __global__ void __launch_bounds__(B2F_RANK_THREADS, 1)
                 const uint32_t xs_lane = xs_addr + (uint32_t)t * B2F_RANK_XS_BYTES + (uint32_t)lane * 4u;
                 double acc = 0.0;
                 for (int g = u - t * groups; g < g_end; ++g)
-                    rank_walk_group<D, U>(forest_addr + (uint32_t)(g * U) * p.tree_stride, p.tree_stride, xs_lane, p.mul_two, p.mul_64k, p.add_64k, acc);
+                    rank_walk_group_head<D, U>(forest_addr + (uint32_t)(g * U) * p.tree_stride, head_addr + (uint32_t)g * (12u * U), p.tree_stride,
+                                               xs_lane, p.mul_two, p.mul_64k, p.add_64k, acc);
                 partial[(warp + t) * 32 + lane] = acc; /* slot (warp + tile) is unique to this (warp, tile) segment */
                 u = t * groups + g_end;
             }
         }
         __syncthreads();
+        RANK_TRACE(RT_WALKED);
+        /* the first global store: the previous launch in the stream may still read these outputs (its rows) or write them.
+         * Rows and forest were read before this point, which is safe because the host never lets a launch with programmatic
+         * serialization read rows that an earlier rank launch of its programmatic chain writes (rank_launch_pdl), and the rank
+         * kernel is the only kernel that triggers its dependents early (griddepcontrol.launch_dependents) */
+        pdl_wait();
+        RANK_TRACE(RT_WAIT);
 
         /* ---- phase 3: one thread per row: partials in warp order -> aggregate -> store ---- */
         for (int r = tid; r < n_rows; r += B2F_RANK_THREADS) {
@@ -291,4 +379,5 @@ __global__ void __launch_bounds__(B2F_RANK_THREADS, 1)
     if constexpr (!STREAM) {
         if (!forest_ready) mbar_wait(&forest_bar[0], 0); /* never retire a CTA while a bulk copy into its shared memory is in flight */
     }
+    RANK_TRACE(RT_EXIT);
 }

@@ -129,7 +129,9 @@ typedef struct b2f_info {
     int32_t rank_smem_bytes; /* dynamic shared memory per CTA of the rank kernel */
     int32_t rank_row_bytes;  /* bytes per ranked row */
     int32_t rank_stream;     /* the rank layout streams through shared memory piece by piece (too large to stay resident) */
-    int32_t reserved2;
+    int32_t rank_last_pdl;   /* the last rank launch went out with programmatic dependent launch (0: its rows overlapped what a
+                                rank launch of the current programmatic chain on its stream writes, or B2F_NO_PDL is set).  "Last" holds for one calling thread: the scorer's workers launch concurrently
+                                on the model's slot streams, like the launch counters above this field is not synchronised */
 } b2f_info;
 
 /* ---- library / device ------------------------------------------------------------------ */
